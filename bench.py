@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our arm (CUDA through the C ABI)
   python bench.py --impl reference --steps K --warmup W    # the reference's CPU algorithm (oracle port)
+  python bench.py ... --dump-outputs DIR                   # also save the last timed step's results as DIR/*.npy
 
 Workload (config.workload): exact brute-force cosine KNN, k=10, batch of 1024 f64 queries per step over a
 10M x 768 f32 corpus (the configuration BASELINE.json's metric is quoted on; it fits one B200).  With N
@@ -289,7 +290,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the HBM-regime table and the int8 peak")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (device-resident path) to DIR as float64 .npy files: "
+                         "knn_rows (global row ids), knn_dist, knn_count; the inputs depend only on the arguments, so "
+                         "two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     rows, dim, batch, k = WORKLOADS[args.workload]
     if args.warmup < 3:
         args.warmup = 3 if args.impl == "ours" else args.warmup
@@ -488,6 +497,13 @@ def main():
     ms_value, wall_value = timed(lambda: run_pipelined(submit_dev, args.warmup, n_batches, True))
     launches = ctx.kernel_launches() - launches0
     stats = col.stats()
+    if args.dump_outputs and rank == 0:
+        # the slot of the last timed batch; nothing reuses d_out before the HBM-regime extras below
+        o = d_out[(n_batches - 1) % DEPTH]
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        # float64 holds every row id (< 2^53) and count exactly
+        for name, t in (("knn_rows", o[0]), ("knn_dist", o[1]), ("knn_count", o[2])):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy().astype(np.float64))
     tick("timed e2e")
     # ---- timed: end to end through the host-buffer plugin call (`e2e`) ----
     ms_e2e, wall_e2e = timed(lambda: run_sync_calls(args.warmup, n_batches))
