@@ -239,7 +239,11 @@ sdb_status sdb_topk_merge_device(sdb_ctx*, uint32_t n_lists, uint32_t nq, uint32
 /* ---- HNSW search: replaces Hnsw::knn_search (idx/trees/hnsw/mod.rs:459-482) called from
  *      HnswIndex::search_graph (idx/trees/hnsw/index.rs:341-364) ------------------------------- */
 /* vectors: n_elems x dim f32 (element id = row).  Layer l adjacency is CSR over element ids;
- * row_ptr[l] has n_elems+1 entries; neighbours keep the stored order (graph.rs:104-125). */
+ * row_ptr[l] has n_elems+1 entries; neighbours keep the stored order (graph.rs:104-125).
+ * Metrics: the F32 typed arithmetic of Distance::calculate (idx/trees/vector.rs:221-410,659-672) for COSINE, EUCLIDEAN,
+ * MANHATTAN, CHEBYSHEV, HAMMING and MINKOWSKI (order: sdb_hnsw_set_minkowski_order), bit-exact except MINKOWSKI, whose
+ * pow() agrees with the platform libm to an ulp or two per call.  PEARSON and JACCARD return SDB_EUNSUPPORTED (the index
+ * keeps the reference's CPU path).  The loaders below accept the same metrics. */
 sdb_status sdb_hnsw_load(sdb_ctx*, uint32_t dim, sdb_metric, uint64_t n_elems, const float* vectors,
                          uint32_t n_layers, const uint64_t* const* row_ptr, const uint32_t* const* col_idx,
                          int64_t entry_point, sdb_hnsw** out);
@@ -277,9 +281,17 @@ sdb_status sdb_hnsw_search_pending(sdb_hnsw*, const float* queries, uint32_t nq,
 /* Distance::calculate for VectorType::F32 vectors (idx/trees/vector.rs:243-289,659-672) applied to vectors that are
  * not part of the graph: the new_vectors of pending updates, which HnswIndex::search_pendings ranks by brute force
  * (hnsw/index.rs:398-404).  query: dim floats, vectors: n x dim floats, out: n doubles (all host memory).  Same
- * arithmetic as the walk kernel (f32 8-lane accumulation, f64 finish). */
+ * arithmetic as the walk kernel (cosine: f32 8-lane accumulation, f64 finish; euclid: sequential f32 sum of squares).
+ * F32 typed metrics served here: cosine / euclid (sdb_hnsw_distance_f32 serves every metric of the walk). */
 sdb_status sdb_vec_distance_f32(sdb_ctx*, sdb_metric, uint32_t dim, const float* query, const float* vectors, uint64_t n,
                                 double* out);
+/* The same for an index: Distance::calculate(query, vector) with the handle's metric and Minkowski order -- what
+ * HnswIndex::search_pendings computes for the new vectors of pending updates (hnsw/index.rs:398-407).  Uses the folds
+ * of the walk kernel, so a vector gets the same distance through the graph and through the pending log. */
+sdb_status sdb_hnsw_distance_f32(sdb_hnsw*, const float* query, const float* vectors, uint64_t n, double* out);
+/* order p of an SDB_MINKOWSKI index (Distance::Minkowski(p)); default 3, as for sdb_corpus_set_minkowski_order.  NaN
+ * returns SDB_EINVAL.  May be called between searches: nothing precomputed depends on it.  Ignored by other metrics. */
+sdb_status sdb_hnsw_set_minkowski_order(sdb_hnsw*, double order);
 
 /* ---- staging: the reference's persisted HNSW state -> device (SURVEY 8a row a14).  These replace the per-key
  *      decode loops of HnswLayer::load (idx/trees/hnsw/layer.rs:526-540, UndirectedGraph::load_node

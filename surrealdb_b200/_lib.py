@@ -29,7 +29,7 @@ ABI_SYMBOLS = [
     "sdb_knn_last_stats", "sdb_knn_submit", "sdb_knn_submit_device", "sdb_knn_wait", "sdb_comm_unique_id",
     "sdb_comm_init_rank", "sdb_comm_size", "sdb_comm_rank", "sdb_ctx_create_multi", "sdb_corpus_set_row_base",
     "sdb_knn_sharded_submit", "sdb_knn_sharded_submit_device", "sdb_knn_sharded_wait", "sdb_knn_sharded_multi",
-    "sdb_corpus_project", "sdb_topk_merge_device", "sdb_hnsw_load", "sdb_hnsw_load_device", "sdb_hnsw_search_device", "sdb_hnsw_select_neighbors_ids", "sdb_hnsw_destroy", "sdb_stage_decode_vectors", "sdb_stage_decode_nodes", "sdb_hnsw_load_staged", "sdb_hnsw_search", "sdb_hnsw_search_filtered", "sdb_hnsw_search_pending", "sdb_vec_distance_f32", "sdb_hnsw_select_neighbors",
+    "sdb_corpus_project", "sdb_topk_merge_device", "sdb_hnsw_load", "sdb_hnsw_load_device", "sdb_hnsw_search_device", "sdb_hnsw_select_neighbors_ids", "sdb_hnsw_destroy", "sdb_stage_decode_vectors", "sdb_stage_decode_nodes", "sdb_hnsw_load_staged", "sdb_hnsw_search", "sdb_hnsw_search_filtered", "sdb_hnsw_search_pending", "sdb_vec_distance_f32", "sdb_hnsw_distance_f32", "sdb_hnsw_set_minkowski_order", "sdb_hnsw_select_neighbors",
     "sdb_graph_load_csr", "sdb_graph_load_csr_shard", "sdb_graph_destroy", "sdb_graph_expand", "sdb_graph_expand_device", "sdb_device_free", "sdb_graph_collect", "sdb_free",
 ]
 
@@ -121,6 +121,8 @@ def lib():
     L.sdb_hnsw_search_filtered.argtypes = [vp, vp, u32, u32, u32, vp, vp, vp, vp, vp]
     L.sdb_hnsw_search_pending.argtypes = [vp, vp, u32, u32, u32, vp, vp, vp, vp, vp]
     L.sdb_vec_distance_f32.argtypes = [vp, i32, u32, vp, vp, u64, vp]
+    L.sdb_hnsw_distance_f32.argtypes = [vp, vp, vp, u64, vp]
+    L.sdb_hnsw_set_minkowski_order.argtypes = [vp, C.c_double]
     L.sdb_hnsw_select_neighbors.argtypes = [vp, vp, u32, i32, u64, u64, vp, vp, u32, u32, i32, vp, vp]
     L.sdb_graph_load_csr.argtypes = [vp, u64, vp, vp, C.POINTER(vp)]
     L.sdb_graph_load_csr_shard.argtypes = [vp, u64, u64, u64, vp, vp, C.POINTER(vp)]

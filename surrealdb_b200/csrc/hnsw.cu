@@ -6,8 +6,10 @@
 //   * candidates popped nearest-first, FIFO among equal distances; stop when nearest candidate > farthest kept
 //   * neighbours visited in STORED order; admitted iff d < f or |w| < ef; w trimmed with pop_last (newest of
 //     the farthest); f re-read after every admission
-//   * distances are the typed-f32 kernels of idx/trees/vector.rs:243-289: cosine = ndarray 8-lane f32 dot and
-//     sums, finished in f64; euclid = sequential f32 sum of squares, f64 sqrt (same op order as the oracle)
+//   * distances are the typed-f32 kernels of idx/trees/vector.rs:221-410: cosine = ndarray 8-lane f32 dot and
+//     sums, finished in f64; euclid = sequential f32 sum of squares, f64 sqrt (same op order as the oracle);
+//     manhattan / chebyshev / hamming = sequential f32 (integer) folds widened to f64; minkowski = sequential f64
+//     sum of |a-b|^p, then ^(1/p).  PEARSON and JACCARD are not served (the index keeps the reference's CPU path).
 // Batched candidate expansion: the <=32 neighbours of the popped candidate are de-duplicated against the
 // per-query visited table with warp-parallel CAS, their vectors are gathered with coalesced transposed loads
 // (one lane per neighbour walks its row in order), and only the admission step is serial.
@@ -17,6 +19,7 @@
 // Algorithmic bytes per query = visited * (4*dim + 4) + expanded * 4*deg, both counters are returned.
 #include <algorithm>
 
+#include "exactmath.cuh"
 #include "internal.cuh"
 #include "rowwalk.cuh"
 
@@ -26,6 +29,7 @@ struct Hnsw {
   Ctx* ctx = nullptr;
   uint32_t dim = 0;
   sdb_metric metric = SDB_EUCLIDEAN;
+  double minkowski_p = 3.0;  // order of SDB_MINKOWSKI (sdb_hnsw_set_minkowski_order); nothing precomputed depends on it
   uint64_t n = 0;
   uint32_t n_layers = 0;
   int64_t entry = -1;
@@ -84,17 +88,72 @@ __global__ void hnsw_sumsq_kernel(const float* __restrict__ vec, uint32_t dim, u
   }
 }
 
-// Distance::calculate for VectorType::F32 (idx/trees/vector.rs:243-289,659-672), one thread per vector: the typed
+// The metrics whose F32 form is ONE fold over the columns in column order (idx/trees/vector.rs), as a per-column
+// policy: step(x, q) takes column c of the element and of the query, finish() widens / finishes to f64.  Only
+// round-to-nearest intrinsics, so nothing is contracted into an FMA (Rust/LLVM does not fuse either).  All four
+// metrics are symmetric bit for bit in (x, q), so calculate(element, query) (the walk, hnsw/elements.rs:128-139) and
+// calculate(query, vector) (the pending log, hnsw/index.rs:407) give the same value.
+template <int METRIC>
+struct RowFold;
+// EUCLID  l2_dist: sequential f32 sum of (a-b)^2, f64 sqrt
+template <>
+struct RowFold<SDB_EUCLIDEAN> {
+  float s = 0.f;
+  __device__ __forceinline__ void step(float x, float q, double) {
+    const float d = __fsub_rn(x, q);
+    s = __fadd_rn(s, __fmul_rn(d, d));
+  }
+  __device__ __forceinline__ double finish(double) const { return __dsqrt_rn((double)s); }
+};
+// MANHATTAN  l1_dist (vector.rs:380): sequential f32 sum of |a-b|, widened.  |.| clears the sign, so a NaN result is
+// positive on the reference's x86-64; it is returned as the canonical 0x7FF8... there (the GPU's own NaN bits differ)
+template <>
+struct RowFold<SDB_MANHATTAN> {
+  float s = 0.f;
+  __device__ __forceinline__ void step(float x, float q, double) { s = __fadd_rn(s, fabsf(__fsub_rn(x, q))); }
+  __device__ __forceinline__ double finish(double) const {
+    return s != s ? __longlong_as_double(0x7FF8000000000000ll) : (double)s;
+  }
+};
+// CHEBYSHEV  linf_dist (vector.rs:221-223): max = 0; if diff > max { max = diff } -- a NaN difference is never taken,
+// so the fold does not depend on the column order
+template <>
+struct RowFold<SDB_CHEBYSHEV> {
+  float m = 0.f;
+  __device__ __forceinline__ void step(float x, float q, double) {
+    const float d = fabsf(__fsub_rn(x, q));
+    if (d > m) m = d;
+  }
+  __device__ __forceinline__ double finish(double) const { return (double)m; }
+};
+// HAMMING  (vector.rs:292-311): count of a != b as FLOAT comparisons (NaN != NaN counts, -0.0 == 0.0 does not)
+template <>
+struct RowFold<SDB_HAMMING> {
+  uint32_t c = 0;
+  __device__ __forceinline__ void step(float x, float q, double) { c += x != q ? 1u : 0u; }
+  __device__ __forceinline__ double finish(double) const { return (double)c; }
+};
+// MINKOWSKI(p)  (vector.rs:389-399): s += |(f64)a - (f64)b|^p in sequential f64, then s^(1/p).  pow() is CUDA's libm
+// here and the platform libm in the reference: an ulp or two apart per call (DESIGN section 8)
+template <>
+struct RowFold<SDB_MINKOWSKI> {
+  ExactAcc a;
+  __device__ __forceinline__ void step(float x, float q, double p) { a.minkowski_step((double)x, (double)q, p); }
+  __device__ __forceinline__ double finish(double p) const { return pow(a.acc, __ddiv_rn(1.0, p)); }
+};
+
+// Distance::calculate for VectorType::F32 (idx/trees/vector.rs:221-410,659-672), one thread per vector: the typed
 // metric of the walk applied to vectors that are NOT part of the graph -- the new_vectors of pending updates that
-// HnswIndex::search_pendings ranks by brute force (hnsw/index.rs:398-404).  Same lane structure as the walk, so a
-// vector gets the same distance whether it is reached through the graph or through the pending log.
-template <bool COSINE>
+// HnswIndex::search_pendings ranks by brute force (hnsw/index.rs:398-404).  Same lane structure and the same folds as
+// the walk, so a vector gets the same distance whether it is reached through the graph or through the pending log.
+// p: the Minkowski order (unused by the other metrics).
+template <int METRIC>
 __global__ void typed_distance_kernel(const float* __restrict__ q, const float* __restrict__ vecs, uint32_t dim, uint64_t n,
-                                      double* __restrict__ out) {
+                                      double p, double* __restrict__ out) {
   const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= n) return;
   const float* a = vecs + r * dim;
-  if (COSINE) {
+  if (METRIC == SDB_COSINE) {
     float p[8] = {0, 0, 0, 0, 0, 0, 0, 0}, pa[8] = {0, 0, 0, 0, 0, 0, 0, 0}, pq[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     uint32_t i = 0;
     for (; i + 8 <= dim; i += 8)
@@ -120,18 +179,16 @@ __global__ void typed_distance_kernel(const float* __restrict__ q, const float* 
     // calculate(a = search.pt, b = vector): dot and the product of norms are symmetric
     out[r] = __dsub_rn(1.0, __ddiv_rn((double)dot, __dmul_rn(na, nb)));
   } else {
-    float s = 0.f;
-    for (uint32_t i = 0; i < dim; i++) {
-      const float d = __fsub_rn(a[i], q[i]);
-      s = __fadd_rn(s, __fmul_rn(d, d));
-    }
-    out[r] = __dsqrt_rn((double)s);
+    RowFold<METRIC == SDB_COSINE ? SDB_EUCLIDEAN : METRIC> f;
+    for (uint32_t i = 0; i < dim; i++) f.step(a[i], q[i], p);
+    out[r] = f.finish(p);
   }
 }
 
 // distance of this lane's row (or NO_ROW) to the query held in shared memory; all 32 lanes must call.
-// Scratch of the distance phase, per warp.  Euclid: a 32 x 33 float transposing tile.  Cosine: 32 compacted row ids +
-// 32 f64 results (the rows are read straight from global memory, see warp_distance<true>).
+// Scratch of the distance phase, per warp.  One lane per row (every metric but cosine): a 32 x 33 float transposing
+// tile.  Cosine: 32 compacted row ids + 32 f64 results (the rows are read straight from global memory, see
+// warp_distance<SDB_COSINE>).
 __host__ __device__ constexpr size_t hn_tile_bytes(bool cosine) { return cosine ? 32 * 4 + 32 * 8 : sizeof(float) * 32 * 33; }
 
 // COSINE.  ndarray's f32 dot (a6; oracle orc_nd_dot_f32) keeps 8 running sums p_j over the columns 8i+j, each one a
@@ -142,10 +199,10 @@ __host__ __device__ constexpr size_t hn_tile_bytes(bool cosine) { return cosine 
 // sector and the 4 rows of a quad 4 sectors, i.e. a request moves as many bytes as a fully coalesced one; no shared-memory
 // transposition, 8 x fewer dependent steps per row than one lane per row (the walk was bound by issue latency: ncu r1,
 // 30 % issue-active at 13 cycles per instruction, ~6.7k instructions per expanded node).
-template <bool COSINE>
+template <int METRIC>
 __device__ __forceinline__ double warp_distance(const float* __restrict__ vec, const double* __restrict__ norm,
                                                 uint32_t dim, uint32_t my_row, const float* s_q, double q_norm,
-                                                float (*tile)[33]);
+                                                float (*tile)[33], double p);
 
 // Cosine keeps the query TRANSPOSED in shared memory: qT[j * qs + i] = q[8i + j] (chain j contiguous), qs = hn_q_stride
 // = 4 mod 32 words so the 8 lanes of a row read 8 different bank groups with one LDS.128 per 4 steps; the < 8 tail
@@ -156,9 +213,9 @@ __host__ __device__ constexpr size_t hn_q_floats(uint32_t dim, bool cosine) {
 }
 
 template <>
-__device__ __forceinline__ double warp_distance<true>(const float* __restrict__ vec, const double* __restrict__ norm,
-                                                      uint32_t dim, uint32_t my_row, const float* s_q, double q_norm,
-                                                      float (*tile)[33]) {
+__device__ __forceinline__ double warp_distance<SDB_COSINE>(const float* __restrict__ vec, const double* __restrict__ norm,
+                                                            uint32_t dim, uint32_t my_row, const float* s_q, double q_norm,
+                                                            float (*tile)[33], double) {
   const uint32_t lane = threadIdx.x & 31u;
   const uint32_t d8 = dim & ~7u, steps = dim >> 3, qs = hn_q_stride(dim);
   uint32_t* ids = reinterpret_cast<uint32_t*>(tile);
@@ -252,14 +309,15 @@ __device__ __forceinline__ double warp_distance<true>(const float* __restrict__ 
   return my_row != NO_ROW ? res[ci] : 0.0;
 }
 
-// EUCLID.  ndarray-stats' l2_dist folds (a-b)^2 strictly sequentially over the columns: one chain per row, so a row
-// stays on ONE lane and the rows of a round are transposed through shared memory (coalesced fetches, 64 columns a step).
-template <>
-__device__ __forceinline__ double warp_distance<false>(const float* __restrict__ vec, const double* __restrict__ norm,
-                                                       uint32_t dim, uint32_t my_row, const float* s_q, double q_norm,
-                                                       float (*tile)[33]) {
+// EUCLID, MANHATTAN, CHEBYSHEV, HAMMING, MINKOWSKI.  Each folds its columns strictly sequentially (RowFold<METRIC>):
+// one chain per row, so a row stays on ONE lane and the rows of a round are transposed through shared memory
+// (coalesced fetches, 64 columns a step).  p: the Minkowski order.
+template <int METRIC>
+__device__ __forceinline__ double warp_distance(const float* __restrict__ vec, const double* __restrict__ norm,
+                                                uint32_t dim, uint32_t my_row, const float* s_q, double q_norm,
+                                                float (*tile)[33], double p) {
   const uint32_t lane = threadIdx.x & 31u;
-  float s = 0.f;
+  RowFold<METRIC> f;
   // Only a handful of the <=32 neighbours of an expanded node are new (6 on average): the valid rows are compacted and
   // handled in rounds of 16; the 32 x 33 float scratch is viewed as 16 rows x (64 columns + 2 padding words), so one
   // step moves 64 columns of every row of the round -- up to 32 independent loads per lane in flight per wait instead
@@ -295,16 +353,13 @@ __device__ __forceinline__ double warp_distance<false>(const float* __restrict__
       __syncwarp();
       if (mine) {
         const uint32_t lim = dim - c0 < 64u ? dim - c0 : 64u;
-        for (uint32_t jj = 0; jj < lim; jj++) {
-          const float d = __fsub_rn(x[jj], s_q[c0 + jj]);
-          s = __fadd_rn(s, __fmul_rn(d, d));
-        }
+        for (uint32_t jj = 0; jj < lim; jj++) f.step(x[jj], s_q[c0 + jj], p);
       }
       __syncwarp();
     }
   }
   if (my_row == NO_ROW) return 0.0;
-  return __dsqrt_rn((double)s);
+  return f.finish(p);
 }
 
 // sorted (ascending key, FIFO inside a key) array insert by the whole warp; entries live in [head, n).  One pass from
@@ -367,10 +422,12 @@ struct HnswParams {
   uint64_t* out_counters;
   uint32_t* overflow;
   const int* cancel;  // mapped host flag (sdb_ctx_cancel): polled before every query
+  double minkowski_p;  // order of SDB_MINKOWSKI
 };
 
-template <bool COSINE, int MINB>
+template <int METRIC, int MINB>
 __global__ void __launch_bounds__(HN_WARPS * 32, MINB) hnsw_search_kernel(HnswParams P) {
+  constexpr bool COSINE = METRIC == SDB_COSINE;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t ccap = P.ccap, wcap = P.ef + 2;
@@ -431,7 +488,7 @@ __global__ void __launch_bounds__(HN_WARPS * 32, MINB) hnsw_search_kernel(HnswPa
     uint32_t n_out = 0;
     if (P.entry >= 0) {
       uint32_t ep = (uint32_t)P.entry;
-      double ep_d = warp_distance<COSINE>(P.vec, P.norm, P.dim, lane == 0 ? ep : NO_ROW, s_q, q_norm, tile);
+      double ep_d = warp_distance<METRIC>(P.vec, P.norm, P.dim, lane == 0 ? ep : NO_ROW, s_q, q_norm, tile, P.minkowski_p);
       ep_d = __shfl_sync(0xffffffffu, ep_d, 0);
       n_visited++;
       for (int32_t layer = (int32_t)P.n_layers - 1; layer >= 0; layer--) {
@@ -494,7 +551,7 @@ __global__ void __launch_bounds__(HN_WARPS * 32, MINB) hnsw_search_kernel(HnswPa
             const uint32_t new_mask = __ballot_sync(0xffffffffu, is_new);
             if (!new_mask) continue;
             n_visited += __popc(new_mask);
-            const double d = warp_distance<COSINE>(P.vec, P.norm, P.dim, is_new ? nb : NO_ROW, s_q, q_norm, tile);
+            const double d = warp_distance<METRIC>(P.vec, P.norm, P.dim, is_new ? nb : NO_ROW, s_q, q_norm, tile, P.minkowski_p);
             // admission in stored order                                     layer.rs:205-217
             uint32_t m = new_mask;
             while (m) {
@@ -744,7 +801,32 @@ using namespace sdb;
 
 extern "C" void sdb_hnsw_destroy(sdb_hnsw* h);
 
-// common tail of the loaders: per-layer pointer tables + cached |x|^2
+// the metrics the walk serves (F32 typed arithmetic): COSINE (8 lanes per row), EUCLIDEAN, MANHATTAN, CHEBYSHEV, HAMMING
+// and MINKOWSKI (one lane per row).  PEARSON and JACCARD are similarities used as distances; the reference's own HNSW
+// tests leave them disabled (idx/trees/hnsw/mod.rs:752-791) and Jaccard's F32 form is asymmetric in its arguments, so
+// indexes declared with them keep the reference's CPU path.
+static sdb_status hnsw_check_metric(sdb_metric metric, const char* what) {
+  switch (metric) {
+    case SDB_COSINE:
+    case SDB_EUCLIDEAN:
+    case SDB_MANHATTAN:
+    case SDB_CHEBYSHEV:
+    case SDB_HAMMING:
+    case SDB_MINKOWSKI:
+      return SDB_OK;
+    case SDB_PEARSON:
+    case SDB_JACCARD:
+      set_error("%s: %s is a similarity used as a distance and is not implemented on the GPU walk (the index keeps the "
+                "reference's CPU path)", what, metric == SDB_PEARSON ? "PEARSON" : "JACCARD");
+      return SDB_EUNSUPPORTED;
+    default:
+      set_error("%s: metric %d not implemented on the GPU path", what, (int)metric);
+      return SDB_EUNSUPPORTED;
+  }
+}
+
+// common tail of the loaders: per-layer pointer tables + cached |x|^2 (cosine / euclid only: the other metrics need no
+// per-element precomputation)
 static sdb_status hnsw_finish(sdb_hnsw* h, sdb_hnsw** out) {
   Ctx* ctx = h->ctx;
   cudaStream_t st = ctx->stream;
@@ -759,7 +841,7 @@ static sdb_status hnsw_finish(sdb_hnsw* h, sdb_hnsw** out) {
   if (cudaMemcpyAsync(h->d_rp, h->rp.data(), sizeof(void*) * n_layers, cudaMemcpyHostToDevice, st) != cudaSuccess ||
       cudaMemcpyAsync(h->d_ci, h->ci.data(), sizeof(void*) * n_layers, cudaMemcpyHostToDevice, st) != cudaSuccess)
     return fail("layer table copy", SDB_ECUDA);
-  if (h->n) {
+  if (h->n && (h->metric == SDB_COSINE || h->metric == SDB_EUCLIDEAN)) {
     if (cudaMalloc(&h->d_norm, sizeof(double) * h->n) != cudaSuccess) return fail("norms", SDB_ENOMEM);
     hnsw_sumsq_kernel<<<(unsigned)((h->n * 8 + 127) / 128), 128, 0, st>>>(h->d_vec, h->dim, h->n, h->d_sumsq, h->d_norm);
     count_launch(ctx);
@@ -793,9 +875,9 @@ sdb_status sdb_hnsw_load(sdb_ctx* ctx, uint32_t dim, sdb_metric metric, uint64_t
   if (!ctx || !out || dim == 0 || dim > 65535 || n_elems >= 0xFFFFFFF0ull || (n_elems && !vectors) || !n_layers ||
       !row_ptr || !col_idx || entry_point >= (int64_t)n_elems)
     return SDB_EINVAL;
-  if (metric != SDB_COSINE && metric != SDB_EUCLIDEAN) {
-    set_error("hnsw: metric %d not implemented on the GPU path", (int)metric);
-    return SDB_EUNSUPPORTED;
+  {
+    const sdb_status mrc = hnsw_check_metric(metric, "sdb_hnsw_load");
+    if (mrc != SDB_OK) return mrc;
   }
   *out = nullptr;
   std::lock_guard<std::mutex> guard(ctx->mu);
@@ -842,9 +924,9 @@ sdb_status sdb_hnsw_load_device(sdb_ctx* ctx, uint32_t dim, sdb_metric metric, u
   if (!ctx || !out || dim == 0 || dim > 65535 || n_elems >= 0xFFFFFFF0ull || (n_elems && !d_vectors) || !n_layers ||
       !d_row_ptr || !d_col_idx || entry_point >= (int64_t)n_elems)
     return SDB_EINVAL;
-  if (metric != SDB_COSINE && metric != SDB_EUCLIDEAN) {
-    set_error("hnsw: metric %d not implemented on the GPU path", (int)metric);
-    return SDB_EUNSUPPORTED;
+  {
+    const sdb_status mrc = hnsw_check_metric(metric, "sdb_hnsw_load_device");
+    if (mrc != SDB_OK) return mrc;
   }
   *out = nullptr;
   std::lock_guard<std::mutex> guard(ctx->mu);
@@ -878,9 +960,9 @@ sdb_status sdb_hnsw_load_staged(sdb_ctx* ctx, uint32_t dim, sdb_metric metric, u
   if (!ctx || !out || dim == 0 || dim > 65535 || n_elems >= 0xFFFFFFF0ull || !n_layers || !node_blob || !node_off ||
       !node_ids || !n_nodes || entry_point >= (int64_t)n_elems || (n_vec && (!vec_blob || !vec_off)))
     return SDB_EINVAL;
-  if (metric != SDB_COSINE && metric != SDB_EUCLIDEAN) {
-    set_error("hnsw: metric %d not implemented on the GPU path", (int)metric);
-    return SDB_EUNSUPPORTED;
+  {
+    const sdb_status mrc = hnsw_check_metric(metric, "sdb_hnsw_load_staged");
+    if (mrc != SDB_OK) return mrc;
   }
   *out = nullptr;
   // The walk kernels implement the reference's typed metrics for VectorType::F32 only (idx/trees/vector.rs:243-289
@@ -1067,8 +1149,17 @@ static sdb_status hnsw_search_impl(sdb_hnsw* h, const float* queries, uint32_t n
   }
   // cosine: 8 lanes per row keep ~16 loads in flight per lane; 80 registers (6 blocks per SM) holds that without spills
   const int occ = getenv("SDB_HNSW_OCC") ? atoi(getenv("SDB_HNSW_OCC")) : 6;  // measured r2 (1M x 768, ef 64): 6 -> 1.40M QPS, 4 -> 1.32M, 8 -> 1.02M (spills)
-  auto kern = h->metric == SDB_COSINE ? (occ >= 8 ? hnsw_search_kernel<true, 8> : occ <= 4 ? hnsw_search_kernel<true, 4> : hnsw_search_kernel<true, 6>)
-                                      : hnsw_search_kernel<false, 1>;
+  void (*kern)(HnswParams);
+  switch (h->metric) {
+    case SDB_COSINE:
+      kern = occ >= 8 ? hnsw_search_kernel<SDB_COSINE, 8> : occ <= 4 ? hnsw_search_kernel<SDB_COSINE, 4> : hnsw_search_kernel<SDB_COSINE, 6>;
+      break;
+    case SDB_MANHATTAN: kern = hnsw_search_kernel<SDB_MANHATTAN, 1>; break;
+    case SDB_CHEBYSHEV: kern = hnsw_search_kernel<SDB_CHEBYSHEV, 1>; break;
+    case SDB_HAMMING: kern = hnsw_search_kernel<SDB_HAMMING, 1>; break;
+    case SDB_MINKOWSKI: kern = hnsw_search_kernel<SDB_MINKOWSKI, 1>; break;
+    default: kern = hnsw_search_kernel<SDB_EUCLIDEAN, 1>; break;  // the loaders admit no other metric
+  }
   SDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   // the walk gets nothing from L1 (0.7 % hit rate): give the whole array to shared memory, or the driver's default
   // carve-out (135 KB) caps the kernel at 5 blocks per SM
@@ -1154,6 +1245,7 @@ static sdb_status hnsw_search_impl(sdb_hnsw* h, const float* queries, uint32_t n
   P.out_count = d_cnt;
   P.out_counters = d_ctr;
   P.overflow = d_ovf;
+  P.minkowski_p = h->minkowski_p;
   kern<<<grid, HN_WARPS * 32, smem, st>>>(P);
   count_launch(ctx);
   h->gen += gens_per_warp * n_tables;
@@ -1193,14 +1285,10 @@ static sdb_status hnsw_search_impl(sdb_hnsw* h, const float* queries, uint32_t n
   return SDB_OK;
 }
 
-sdb_status sdb_vec_distance_f32(sdb_ctx* ctx, sdb_metric metric, uint32_t dim, const float* query, const float* vectors,
-                                uint64_t n, double* out) {
-  if (!ctx || !dim || (n && (!query || !vectors || !out))) return SDB_EINVAL;
-  if (metric != SDB_COSINE && metric != SDB_EUCLIDEAN) {
-    set_error("sdb_vec_distance_f32: metric %d not implemented on the GPU path", (int)metric);
-    return SDB_EUNSUPPORTED;
-  }
-  if (n == 0) return SDB_OK;
+// Distance::calculate(query, vector) for n host vectors on the context's stream (sdb_vec_distance_f32 /
+// sdb_hnsw_distance_f32); the metric has been validated by the caller
+static sdb_status typed_distances(Ctx* ctx, sdb_metric metric, double p, uint32_t dim, const float* query,
+                                  const float* vectors, uint64_t n, double* out, const char* what) {
   std::lock_guard<std::mutex> guard(ctx->mu);
   SDB_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
@@ -1212,8 +1300,15 @@ sdb_status sdb_vec_distance_f32(sdb_ctx* ctx, sdb_metric metric, uint32_t dim, c
     SDB_CUDA(cudaMallocAsync(&d_o, sizeof(double) * n, st));
     SDB_CUDA(cudaMemcpyAsync(d_q, query, sizeof(float) * dim, cudaMemcpyHostToDevice, st));
     SDB_CUDA(cudaMemcpyAsync(d_v, vectors, sizeof(float) * n * dim, cudaMemcpyHostToDevice, st));
-    if (metric == SDB_COSINE) typed_distance_kernel<true><<<(unsigned)((n + 127) / 128), 128, 0, st>>>(d_q, d_v, dim, n, d_o);
-    else typed_distance_kernel<false><<<(unsigned)((n + 127) / 128), 128, 0, st>>>(d_q, d_v, dim, n, d_o);
+    const unsigned grid = (unsigned)((n + 127) / 128);
+    switch (metric) {
+      case SDB_COSINE: typed_distance_kernel<SDB_COSINE><<<grid, 128, 0, st>>>(d_q, d_v, dim, n, p, d_o); break;
+      case SDB_MANHATTAN: typed_distance_kernel<SDB_MANHATTAN><<<grid, 128, 0, st>>>(d_q, d_v, dim, n, p, d_o); break;
+      case SDB_CHEBYSHEV: typed_distance_kernel<SDB_CHEBYSHEV><<<grid, 128, 0, st>>>(d_q, d_v, dim, n, p, d_o); break;
+      case SDB_HAMMING: typed_distance_kernel<SDB_HAMMING><<<grid, 128, 0, st>>>(d_q, d_v, dim, n, p, d_o); break;
+      case SDB_MINKOWSKI: typed_distance_kernel<SDB_MINKOWSKI><<<grid, 128, 0, st>>>(d_q, d_v, dim, n, p, d_o); break;
+      default: typed_distance_kernel<SDB_EUCLIDEAN><<<grid, 128, 0, st>>>(d_q, d_v, dim, n, p, d_o); break;
+    }
     count_launch(ctx);
     SDB_CUDA(cudaGetLastError());
     SDB_CUDA(cudaMemcpyAsync(out, d_o, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
@@ -1224,10 +1319,39 @@ sdb_status sdb_vec_distance_f32(sdb_ctx* ctx, sdb_metric metric, uint32_t dim, c
   if (d_v) cudaFreeAsync(d_v, st);
   if (d_o) cudaFreeAsync(d_o, st);
   if (cudaStreamSynchronize(st) != cudaSuccess && rc == SDB_OK) {
-    set_error("sdb_vec_distance_f32: %s", cudaGetErrorString(cudaGetLastError()));
+    set_error("%s: %s", what, cudaGetErrorString(cudaGetLastError()));
     return SDB_ECUDA;
   }
   return rc;
+}
+
+sdb_status sdb_vec_distance_f32(sdb_ctx* ctx, sdb_metric metric, uint32_t dim, const float* query, const float* vectors,
+                                uint64_t n, double* out) {
+  if (!ctx || !dim || (n && (!query || !vectors || !out))) return SDB_EINVAL;
+  if (metric != SDB_COSINE && metric != SDB_EUCLIDEAN) {
+    set_error("sdb_vec_distance_f32: metric %d not implemented on the GPU path", (int)metric);
+    return SDB_EUNSUPPORTED;
+  }
+  if (n == 0) return SDB_OK;
+  return typed_distances(ctx, metric, 3.0, dim, query, vectors, n, out, "sdb_vec_distance_f32");
+}
+
+sdb_status sdb_hnsw_distance_f32(sdb_hnsw* h, const float* query, const float* vectors, uint64_t n, double* out) {
+  if (!h || (n && (!query || !vectors || !out))) return SDB_EINVAL;
+  if (n == 0) return SDB_OK;
+  double p;
+  {
+    std::lock_guard<std::mutex> guard(h->mu);
+    p = h->minkowski_p;
+  }
+  return typed_distances(h->ctx, h->metric, p, h->dim, query, vectors, n, out, "sdb_hnsw_distance_f32");
+}
+
+sdb_status sdb_hnsw_set_minkowski_order(sdb_hnsw* h, double order) {
+  if (!h || !(order == order)) return SDB_EINVAL;
+  std::lock_guard<std::mutex> guard(h->mu);  // a search in flight keeps the order it started with
+  h->minkowski_p = order;
+  return SDB_OK;
 }
 
 sdb_status sdb_hnsw_search(sdb_hnsw* h, const float* queries, uint32_t nq, uint32_t k, uint32_t ef, uint64_t* out_elems,

@@ -9,6 +9,10 @@
                                       (idx/trees/knn.rs:363-437): final order (distance, VectorId), <= k
   HnswIndex.add_pending(...)          the Hp log (VectorPendingUpdate, hnsw/mod.rs:88-113) as the Rust shim streams it
   HnswIndex.check_state(state)        Hnsw::check_state (hnsw/mod.rs:187-224): is the device copy still current?
+
+Metrics (DIST of the index): COSINE, EUCLIDEAN, MANHATTAN, CHEBYSHEV, HAMMING and MINKOWSKI (minkowski_order, default
+3) in the reference's F32 typed arithmetic.  PEARSON and JACCARD raise SdbError(SDB_EUNSUPPORTED): such indexes keep
+the reference's CPU path.
 """
 import ctypes as C
 
@@ -39,10 +43,11 @@ class KnnResultBuilder:
 
 
 class HnswIndex:
-    def __init__(self, ctx, vectors, layers, entry_point, metric="EUCLIDEAN", elem_docs=None):
+    def __init__(self, ctx, vectors, layers, entry_point, metric="EUCLIDEAN", elem_docs=None, minkowski_order=3.0):
         """vectors (n, dim) f32; layers = [(row_ptr u64[n+1], col_idx u32[e]), ...] layer 0 first;
         elem_docs: optional list of doc-id lists per element (identical vectors share one element:
-        hnsw/docs.rs:161-176); default = one doc per element with the same id."""
+        hnsw/docs.rs:161-176); default = one doc per element with the same id.  minkowski_order: the p of
+        DIST MINKOWSKI p (ignored by the other metrics)."""
         vec = np.ascontiguousarray(vectors, np.float32)
         self.n, self.dim = vec.shape
         self.ctx, self.metric = ctx, metric.upper()
@@ -57,9 +62,10 @@ class HnswIndex:
         self.h = C.c_void_p()
         L.check(L.lib().sdb_hnsw_load(ctx.h, self.dim, L.METRIC[self.metric], self.n, C.c_void_p(vec.ctypes.data), nl,
                                       RP, CI, int(entry_point), C.byref(self.h)))
+        self.set_minkowski_order(minkowski_order)
 
     @classmethod
-    def from_device(cls, ctx, x_dev, layers_dev, entry_point, metric="EUCLIDEAN", elem_docs=None):
+    def from_device(cls, ctx, x_dev, layers_dev, entry_point, metric="EUCLIDEAN", elem_docs=None, minkowski_order=3.0):
         """wraps device-resident vectors and CSR layers WITHOUT copying them (sdb_hnsw_load_device): x_dev is a torch CUDA
         float32 (n, dim) tensor, layers_dev = [(row_ptr int64 (n+1), col_idx int32)] layer 0 first.  The tensors must
         stay alive (they are kept on the object)."""
@@ -74,10 +80,12 @@ class HnswIndex:
         self.h = C.c_void_p()
         L.check(L.lib().sdb_hnsw_load_device(ctx.h, self.dim, L.METRIC[self.metric], self.n, C.c_void_p(x_dev.data_ptr()), nl,
                                              RP, CI, int(entry_point), C.byref(self.h)))
+        self.set_minkowski_order(minkowski_order)
         return self
 
     @classmethod
-    def from_kv(cls, ctx, dim, state_value, he_items, hn_items_per_layer, metric="EUCLIDEAN", elem_docs=None):
+    def from_kv(cls, ctx, dim, state_value, he_items, hn_items_per_layer, metric="EUCLIDEAN", elem_docs=None,
+                minkowski_order=3.0):
         """Loads the index straight from raw KV values (staging.py): `state_value` = the Hs value, `he_items` =
         [(element id, He value)], `hn_items_per_layer[l]` = [(node id, Hn value)] of layer l (0 first), each in key
         order.  Decoding happens on the GPU (sdb_hnsw_load_staged).  Mirrors Hnsw::check_state + HnswLayer::load
@@ -107,7 +115,13 @@ class HnswIndex:
                                              C.c_void_p(vo.ctypes.data), C.c_void_p(vi.ctypes.data), len(he_items), nl,
                                              NB, NO, NI, NN, ep, C.byref(self.h), C.byref(bad)))
         self.n_bad = bad.value
+        self.set_minkowski_order(minkowski_order)
         return self
+
+    def set_minkowski_order(self, order):
+        """the p of Distance::Minkowski(p) (sdb_hnsw_set_minkowski_order); may change between searches.  NaN raises
+        SdbError(SDB_EINVAL).  Ignored by the other metrics."""
+        L.check(L.lib().sdb_hnsw_set_minkowski_order(self.h, float(order)))
 
     # ---- freshness: layer versions (Hs) and the pending log (Hp) ---------------------------------------------------
     def check_state(self, state_value):
@@ -135,12 +149,13 @@ class HnswIndex:
         return (0, int(vid)) if isinstance(vid, (int, np.integer)) else (1, vid)
 
     def _typed_distances(self, query, vectors):
-        """Distance::calculate(&search.pt, &vector) for F32 vectors, on the GPU (sdb_vec_distance_f32)"""
+        """Distance::calculate(&search.pt, &vector) for F32 vectors with the index's metric and Minkowski order, on the
+        GPU (sdb_hnsw_distance_f32)"""
         q = np.ascontiguousarray(query, np.float32)
         v = np.ascontiguousarray(vectors, np.float32).reshape(-1, self.dim)
         out = np.zeros(v.shape[0], np.float64)
-        L.check(L.lib().sdb_vec_distance_f32(self.ctx.h, L.METRIC[self.metric], self.dim, C.c_void_p(q.ctypes.data),
-                                             C.c_void_p(v.ctypes.data), v.shape[0], C.c_void_p(out.ctypes.data)))
+        L.check(L.lib().sdb_hnsw_distance_f32(self.h, C.c_void_p(q.ctypes.data), C.c_void_p(v.ctypes.data), v.shape[0],
+                                              C.c_void_p(out.ctypes.data)))
         return out
 
     def search_graph(self, queries, k, ef, counters=False, truthy=None, all_docs_pending=None):
